@@ -16,16 +16,22 @@ One "step" = one full pass of the hot path over the rank's lineitem partition:
            cores) -- the reference's Rust/DataFusion path cannot be built in this image (no Rust).
 
 Launch: python bench.py [--gpus N --steps K --warmup W]   (torchrun for N>1, one rank per GPU)
+`--dump-outputs DIR`: after the timed steps, the Q1 result of the last timed step as DIR/<output>.npy (float64), for comparing
+           two builds on the same seeded inputs.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
 import tempfile
 import threading
 import time
+
+sys.dont_write_bytecode = True   # the source tree may be read-only: nothing is written into it
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "datafusion-comet_b200")):
@@ -334,6 +340,21 @@ def setup(args):
                 max_over_ranks=max_over_ranks, sum_over_ranks=sum_over_ranks)
 
 
+def private_jit_cache():
+    """Kernels compiled at run time (range-specialised variants of the pipelines) are cached in a temporary directory rather
+    than next to the library, so the source tree stays untouched; the cubins build() compiled are linked in and not compiled
+    again."""
+    if os.environ.get("CB200_CACHE_DIR"):
+        return
+    shipped = os.path.join(ROOT, "datafusion-comet_b200", ".jitcache")
+    d = tempfile.mkdtemp(prefix="cb200_jitcache_")
+    atexit.register(shutil.rmtree, d, True)
+    if os.path.isdir(shipped):
+        for f in os.listdir(shipped):
+            os.symlink(os.path.join(shipped, f), os.path.join(d, f))
+    os.environ["CB200_CACHE_DIR"] = d
+
+
 def timed_region(env, sampler, step_fn, warmup, steps):
     """W untimed steps, then exactly K steps between barrier + synchronize on both sides; max over ranks."""
     import gc
@@ -444,6 +465,18 @@ Q1_OUT = ["sum_qty", "sum_base_price", "sum_disc_price", "sum_charge", "avg_qty"
 Q1_SCALE = [2, 2, 4, 6, 6, 6, 6]
 
 
+def q1_dump(res, out_dir):
+    """The Final plan's result rows, ordered by (l_returnflag, l_linestatus), one float64 array per output column: the flags
+    as their character codes, decimals and doubles by value, count_order as a number."""
+    import numpy as np
+    rows = sorted(res.to_pylist(), key=lambda r: (r["col_0"], r["col_1"]))
+    os.makedirs(out_dir, exist_ok=True)
+    names = ["l_returnflag", "l_linestatus"] + Q1_OUT + ["count_order"]
+    for j, name in enumerate(names):
+        v = [ord(r[f"col_{j}"]) if j < 2 else float(r[f"col_{j}"]) for r in rows]
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 def q1_compare(tpch, res, expected):
     """res: the Final plan's Arrow table; expected: {group index: dict}.  True iff all eight outputs of every group agree."""
     got = {(r["col_0"], r["col_1"]): r for r in res.to_pylist()}
@@ -500,6 +533,8 @@ def workload_q1(args, env):
     pipe_launches = sum(o[1]["pipeline_launches"] for o in outs)
     launches = sum(o[1]["kernel_launches"] + (o[2]["kernel_launches"] if o[2] else 0) for o in outs)
     res = outs[-1][0]
+    if rank == 0 and args.dump_outputs:
+        q1_dump(res, args.dump_outputs)
 
     # ---- checks (outside the timed region) ---------------------------------------------------------------------------------------
     # (1) every output of every group at FULL size against exact torch int64 arithmetic (rank 0's partition; N = 1 only: the final
@@ -930,7 +965,12 @@ def main():
                     help="all = writer default of Spark/parquet-mr and pyarrow (dictionary-encode every column, PLAIN fallback); flags = PLAIN numerics")
     ap.add_argument("--parquet-compression", default="NONE", choices=["NONE", "SNAPPY"])
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the Q1 result of the last timed step as DIR/<output>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "q1"):
+        ap.error("--dump-outputs writes the result of the b200 q1 workload")
     if os.environ.get("CB200_BENCH_TRACE_S"):          # debugging aid: dump every thread's Python stack every N seconds to stderr
         import faulthandler
         faulthandler.dump_traceback_later(float(os.environ["CB200_BENCH_TRACE_S"]), repeat=True)
@@ -939,6 +979,7 @@ def main():
     if args.impl == "reference":
         reference_arm(args, rank, world)
         return
+    private_jit_cache()
     env = setup(args)
     if args.workload == "q1":
         workload_q1(args, env)

@@ -4,8 +4,8 @@ This is the stand-in for the JVM side (`QueryPlanSerde.scala`, `operators.scala:
 *produces* `spark.spark_operator.Operator` bytes: tests and bench.py build the same messages the
 Spark plugin would send through `Native.createPlan` (`Native.scala:60-79`).  Field numbers are the
 reference's (native/proto/src/proto/{operator,expr,literal,types,partitioning}.proto); the test
-`tests/test_proto.py::test_field_numbers_match_reference` re-reads the .proto files when the
-reference tree is present and checks every number used here.
+`tests/test_proto.py::test_field_numbers_match_reference` checks every number used here against
+the numbers recorded from those files in tests/golden/proto_field_numbers.json.
 
 No protoc / generated code: the wire format is five rules (varint, fixed64, length-delimited,
 fixed32, tags), written out below.

@@ -1,41 +1,16 @@
 """The hand-written plan encoder/decoder must use the reference's field numbers."""
+import json
 import os
-import re
 
-import pytest
-
-REF = "/root/reference/native/proto/src/proto"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "proto_field_numbers.json")
 
 
-def parse_proto(path):
-    """{message_or_oneof_scope: {field_name: number}} with nested messages flattened by simple name."""
-    txt = re.sub(r"//[^\n]*", "", open(path).read())
-    out = {}
-    stack = []
-    for tok in re.finditer(r"(message|enum|oneof)\s+(\w+)\s*\{|\}|(?:repeated\s+|optional\s+)?[\w.<>, ]+?\s+(\w+)\s*=\s*(\d+)\s*(?:\[[^\]]*\])?;|(\w+)\s*=\s*(-?\d+)\s*;", txt):
-        if tok.group(1):
-            stack.append((tok.group(1), tok.group(2)))
-            if tok.group(1) != "oneof":
-                out.setdefault(tok.group(2), {})
-        elif tok.group(0) == "}":
-            if stack:
-                stack.pop()
-        else:
-            name, num = (tok.group(3), tok.group(4)) if tok.group(3) else (tok.group(5), tok.group(6))
-            owner = next((n for k, n in reversed(stack) if k != "oneof"), None)
-            if owner:
-                out[owner][name] = int(num)
-    return out
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted (GPU box)")
 def test_field_numbers_match_reference():
+    """Every number the encoder uses, against the reference's .proto files as recorded by tools/proto_field_numbers.py."""
+    with open(GOLDEN) as f:
+        ref = json.load(f)
     from comet_b200 import proto as P
-    expr = parse_proto(os.path.join(REF, "expr.proto"))
-    op = parse_proto(os.path.join(REF, "operator.proto"))
-    types = parse_proto(os.path.join(REF, "types.proto"))
-    lit = parse_proto(os.path.join(REF, "literal.proto"))
-    part = parse_proto(os.path.join(REF, "partitioning.proto"))
+    expr, op, types, lit, part = (ref[k] for k in ("expr", "operator", "types", "literal", "partitioning"))
     for k, v in P.EXPR_FIELD.items():
         assert expr["Expr"][k] == v, k
     for k, v in P.AGG_FIELD.items():
